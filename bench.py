@@ -213,7 +213,7 @@ def shared_volume_leg(kb, torch, args, world, rank, local, device, dev_depth, de
     if world > 1:
         from kintinuous_b200 import mgpu
         mgpu.connect(trk)
-    steps = max(20, min(args.steps, 100))
+    steps = args.steps
     prewarm = 40
 
     def run(k, i):
@@ -312,6 +312,50 @@ def run_reference(args, world, rank, local):
     print(json.dumps(line), flush=True)
 
 
+DUMP_LIMIT_BYTES = 64_000_000        # everything --dump-outputs writes, all files together
+DUMP_MAP_PIXELS = 640 * 480          # a larger frame's model maps are dumped at a fixed, seeded sample of this many pixels
+DUMP_VOXELS = 2_000_000
+
+
+def _map_with_mask(m):
+    """A vertex / normal map (x, y, z planes first) as the reference stores it marks a pixel without a surface with NaN in its x plane
+    (its y / z planes keep stale values).  Dumped as the map with those pixels zeroed in all three planes plus a 0 / 1 mask of the
+    valid pixels, so every value is finite and two runs compare element for element."""
+    valid = ~np.isnan(m[0])
+    m = np.where(valid[None], m, np.float32(0)).astype(np.float32)
+    return m, valid.astype(np.float32)
+
+
+def dump_outputs(out_dir, trk, pose, zslab):
+    """What the timed path computed in its last step, as float32 / float64 .npy files of at most DUMP_LIMIT_BYTES together (about 26 MB
+    at 640x480): the pose that kt_process_frame_device returned, the model vertex / normal maps the frame left for the next one (with
+    their validity masks), and the TSDF value and weight of a fixed, seeded sample of voxels.  The samples are drawn with seed 0 from
+    the frame size and the volume side alone, so every run with the same arguments dumps the same pixels and voxels.  In the z-slab
+    mode rank 0 holds only its own storage planes of the volume, so the voxels are drawn from those (Tracker.export_owned)."""
+    R, t, global_t, wrap = pose.as_tuple()
+    out = {"pose_R": R, "pose_t": t, "pose_global_t": global_t, "pose_voxel_wrap": wrap.astype(np.float64)}
+    npix = trk.cfg.rows * trk.cfg.cols
+    pix = np.sort(np.random.default_rng(0).choice(npix, DUMP_MAP_PIXELS, replace=False)) if npix > DUMP_MAP_PIXELS else None
+    for name, which in (("model_vmap", 2), ("model_nmap", 3)):
+        m = trk.download_map(which, 0)
+        if pix is not None:
+            m = m.reshape(3, -1)[:, pix]
+        out[name], out[name + "_valid"] = _map_with_mask(m)
+    tsdf, color = trk.export_owned() if zslab else trk.export_volume()
+    idx = np.sort(np.random.default_rng(0).choice(tsdf.size, min(DUMP_VOXELS, tsdf.size), replace=False))
+    out["volume_sample_tsdf"] = tsdf.reshape(-1)[idx].astype(np.float32)
+    out["volume_sample_weight"] = color.reshape(-1, 4)[idx, 3].astype(np.float32)
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    for name, a in out.items():
+        if not np.isfinite(a).all():
+            raise RuntimeError(f"--dump-outputs: {name} is not finite")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -328,7 +372,12 @@ def main():
     ap.add_argument("--vol", type=int, default=VOL)
     ap.add_argument("--scale", type=int, default=1, help="image scale: 1 = 640x480 (configs 1-3), 2 = 1280x960 (configs[4])")
     ap.add_argument("--odometry", type=int, default=0, help="0 ICP (configs[1]), 2 ICP+RGB-D (configs[2])")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed device path computed in its last step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.shared_only or args.impl == "reference"):
+        ap.error("--dump-outputs dumps the b200 arm's main timed path; it does not apply with --shared-only or --impl reference")
     global ROWS, COLS, P_LEVELS, N_INPUT_FRAMES
     if args.scale != 1:
         ROWS, COLS = 480 * args.scale, 640 * args.scale
@@ -369,21 +418,23 @@ def main():
                             rank=rank if zslab else 0, world=world if zslab else 1)
 
     def run(tracker, use_host, steps, start):
+        """Process `steps` frames from frame index `start`; returns the next index and the pose of the last frame."""
         i = start
+        p = None
         for _ in range(steps):
             j = pingpong(i, n)
             jn = pingpong(i + 1, n)
             # kt_prefetch_frame (public API hint): the next frame's copy and pose-independent front end overlap this frame's fusion
             if use_host:
-                tracker.process_frame(pin_depth[j].data_ptr(), pin_rgb[j].data_ptr(), i)
+                p = tracker.process_frame(pin_depth[j].data_ptr(), pin_rgb[j].data_ptr(), i)
                 if not args.no_prefetch:
                     tracker.prefetch_frame(pin_depth[jn].data_ptr(), pin_rgb[jn].data_ptr())
             else:
-                tracker.process_frame_device(dev_depth[j], dev_rgb[j], i)
+                p = tracker.process_frame_device(dev_depth[j], dev_rgb[j], i)
                 if not args.no_prefetch:
                     tracker.prefetch_frame(dev_depth[jn], dev_rgb[jn])
             i += 1
-        return i
+        return i, p
 
     results = {}
     clocks = None
@@ -395,7 +446,7 @@ def main():
         sampler = ClockSampler(local) if (leg == "device" and rank == 0) else None      # NVML init / child start-up outside the timed region
         # frame 0 + W warm-up frames as the contract asks, preceded by PREWARM more untimed frames: the inputs were rendered on the CPU
         # for seconds with the GPU idle, and W = 3 frames (1 ms) do not bring its clocks and the allocator to steady state
-        i = run(trk, leg == "host", PREWARM + warmup + 1, 0)
+        i, _ = run(trk, leg == "host", PREWARM + warmup + 1, 0)
         torch.cuda.synchronize(); barrier(world)
         if leg == "device" and rank == 0:
             sampler.start()
@@ -403,7 +454,7 @@ def main():
         torch.cuda.synchronize()
         t0 = time.perf_counter()
         trk.span_mark(0)                                    # CUDA events on the tracker's own stream (torch events would not see it)
-        i = run(trk, leg == "host", args.steps, i)
+        i, last = run(trk, leg == "host", args.steps, i)
         trk.span_mark(1)
         dt = trk.span_elapsed_ms() * 1e-3                   # synchronises on the closing event
         torch.cuda.synchronize()
@@ -416,6 +467,8 @@ def main():
             raise RuntimeError("device stopwatch failed")
         dt = max_over_ranks(dt, world, device)
         results[leg] = {"dt": dt, "wall": max_over_ranks(wall, world, device), "launches": l1 - l0}
+        if leg == "device" and args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, trk, last, zslab)
         if leg == "device":
             # stage timers (CUDA events on the tracker's stream) over a few extra frames, outside the timed region
             trk.set_stage_timing(True)

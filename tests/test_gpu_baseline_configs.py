@@ -1,5 +1,6 @@
 """GPU parity at BASELINE.json's OWN configurations -- 640x480 frames into a 512^3 volume, the default -t 14 shift threshold, all three
-odometry modes -- against the reference's CUDA path compiled for VOL=512 (oracle/_ref/libkt_ref_512.so), running live on the same box.
+odometry modes -- against the reference's CUDA path compiled for VOL=512, recorded on a B200 (tools/make_golden_live.py ->
+tests/golden/ref_baseline_512.npz: the reference's poses, its front end and its replay as digests, a sample of its volume).
 
 Three statements per run, each exact or with its tolerance written here:
 
@@ -21,17 +22,22 @@ Three statements per run, each exact or with its tolerance written here:
 2. VOLUME, EXACT.  The sequence-level TSDF bar cannot be "every voxel within 1 LSB of the reference's run": the two trackers' poses differ
    in the 7th digit, which moves a handful of voxel projections across a pixel boundary, and such a voxel fuses a DIFFERENT pixel's depth
    -- its difference is bounded by |D(u,v) - D(u',v')| / mu per frame (a depth edge: the full TSDF range), not by 1 LSB.  What can be
-   demanded exactly is stronger: replay the product's own pose sequence through the REFERENCE's operators (bilateral, createVMap/NMap,
-   scaleDepth + tsdf23, clearVolume*) on a second volume, frame by frame, and require the product's volume -- TSDF, weights AND colours,
-   every voxel, after a real shift -- to be BIT-IDENTICAL to it: 0 LSB.  Pose closeness is statement 1; given the poses, fusion is exact.
+   demanded exactly is stronger: replay the product's own pose sequence through the operators (bilateral, createVMap/NMap, scaleDepth +
+   tsdf23, clearVolume*) on a second volume, frame by frame, and require the product's volume -- TSDF, weights AND colours, every voxel,
+   after a real shift -- to be BIT-IDENTICAL to it: 0 LSB.  Pose closeness is statement 1; given the poses, fusion is exact.  The replay
+   runs the product's operators; that they are the REFERENCE's is checked on the same sequence: the product's operators replaying the
+   pose sequence recorded with the reference must give the reference replay's volume and slabs, digest for digest.
 
 3. SLICES, EXACT.  At each shift the slab the product hands out must equal, as a multiset of 32-byte points, what the reference's
-   extractCloudSlice returns on the replayed volume for the same box (extract.cu:325-419; slab boxes from KintinuousTracker.cpp:675-831).
+   extractCloudSlice returns on the replayed volume for the same box (extract.cu:325-419; slab boxes from KintinuousTracker.cpp:675-831)
+   -- again through the product's extraction operator on the replay, pinned to the reference's by the recorded replay.
 """
 import os
 
 import numpy as np
 import pytest
+
+from conftest import GOLDEN
 
 pytestmark = pytest.mark.gpu
 
@@ -79,57 +85,74 @@ def frames26():
         return [synth.render(k) for k in range(72)]
 
 
-@pytest.mark.parametrize("odometry,nframes", [(0, 72), (2, 22), (1, 26)])
-def test_baseline_config_512_live_replay_exact(built, frames26, odometry, nframes):
+def _replay(frames26, seq, cfg, trunc):
+    """Fuse a pose sequence with the product's OPERATORS (kt_op_*) on a volume of their own.  Per frame: the front end on persistent
+    buffers (Q7 staleness of invalid map pixels), the frame's shift events (slab extraction, clear), integrate.  A row of seq is the
+    tracker's voxel wrap after the frame, then Rinv (9), t (3) and wrap (3) of its integration.  Returns the volume, the final signed
+    voxel wrap and the extracted slabs as (frame, axis, n, canonical points)."""
     import torch
     import kintinuous_b200 as kb
     from kintinuous_b200 import synth
-    from oracle import refbind
-    if not refbind.RefCuda.available(V):
-        pytest.skip("oracle/_ref/libkt_ref_512.so not present")
-    ref = refbind.RefCuda(V)
-    cfg = kb.Config.default(vol=V, odometry=odometry)                  # voxel_shift 14, overlap 2: BASELINE configs[1] / configs[2]
-    assert cfg.voxel_shift == 14 and cfg.overlap == 2
-    mine = kb.Tracker(cfg)
-    rt = ref.tracker(refbind.TrackerConfig.from_kt(cfg))
-    rp = ref.tracker(refbind.TrackerConfig.from_kt(cfg)) if odometry == 0 else None      # ref': 1-LSB perturbed input (statement 1)
+    from oracle.golden import canon_points
+    ops = kb.ops
     intr = np.array(synth.intrinsics(COLS, ROWS), np.float32)
     vs = [SIZE] * 3
-    trunc = mine.trunc_dist
-    assert abs(trunc - rt.trunc_dist) == 0.0
-    # the replay volume and the reference-side front end buffers (persistent: Q7 staleness of invalid map pixels)
     ts = torch.zeros(V ** 3, dtype=torch.int16, device="cuda"); cs = torch.zeros(V ** 3 * 4, dtype=torch.uint8, device="cuda")
-    ref.init_volume(ts, cs)
+    ops.init_volume(ts, cs, V)
     fb = torch.zeros((ROWS, COLS), dtype=torch.int16, device="cuda")
     vm = torch.zeros((3 * ROWS, COLS), dtype=torch.float32, device="cuda"); nm = torch.zeros_like(vm)
     ds = torch.zeros((ROWS, COLS), dtype=torch.float32, device="cuda")
     cap = 3 * ROWS * COLS
     ob = torch.zeros(cap * 32, dtype=torch.uint8, device="cuda")
     cur = [0, 0, 0]                                                     # signed voxelWrap of the replay
-    n_slices = 0
-    slice_points = 0
-    shifted_frames = []
+    slabs = []
+    for k in range(len(seq)):
+        d, c = frames26[k]
+        dd = torch.from_numpy(d.view(np.int16)).cuda(); cc = torch.from_numpy(c).cuda()
+        ops.bilateral(dd, fb, ROWS, COLS); ops.create_vmap(intr, fb, vm, ROWS, COLS); ops.create_nmap(vm, nm, ROWS, COLS)
+        for axis in range(3):                                           # x, then y, then z (.cpp:675-831)
+            n = int(seq[k][axis]) - cur[axis]
+            if n == 0:
+                continue
+            assert abs(n) == cfg.voxel_shift
+            box = shift_box(axis, n, cfg.overlap)
+            cnt = ops.extract_slice(ts, vs, V, ob, cap, vwrap_nonneg(cur), cs, box, 1, tuple(cur))
+            slabs.append((k, axis, n, canon_points(ob[:cnt * 32])))
+            ops.clear_volume(axis, 1 if n < 0 else 0, ts, cs, V, cur[axis], cur[axis] + n)
+            cur[axis] += n
+        Rinv = seq[k][3:12].astype(np.float32).reshape(3, 3); tint = seq[k][12:15].astype(np.float32); wint = [int(x) for x in seq[k][15:18]]
+        assert wint == (vwrap_nonneg(cur) if k > 0 else [0, 0, 0])
+        ops.integrate(dd, ROWS, COLS, intr, vs, Rinv, tint, trunc, ts, cs, V, wint, cc, nm, 1, ds)
+    torch.cuda.synchronize()
+    return ts, cs, cur, slabs
+
+
+@pytest.mark.parametrize("odometry,nframes", [(0, 72), (2, 22), (1, 26)])
+def test_baseline_config_512_live_replay_exact(built, frames26, odometry, nframes):
+    import torch
+    import kintinuous_b200 as kb
+    from oracle.golden import digest, canon_points
+    G = np.load(os.path.join(GOLDEN, "ref_baseline_512.npz"))
+    p = f"o{odometry}_"
+    cfg = kb.Config.default(vol=V, odometry=odometry)                  # voxel_shift 14, overlap 2: BASELINE configs[1] / configs[2]
+    assert cfg.voxel_shift == 14 and cfg.overlap == 2
+    mine = kb.Tracker(cfg)
+    trunc = mine.trunc_dist
+    assert abs(trunc - float(G[p + "trunc"])) == 0.0
+    # K*: first frame where the reference is unstable under a 1-LSB input change (ref' of the module docstring, recorded)
+    horizon = int(G[p + "horizon"]) if odometry == 0 and int(G[p + "horizon"]) >= 0 else None
+    if horizon is not None:
+        print(f"stable horizon K* = {horizon}: the reference moved > 2e-5 m under a 1-LSB change of one depth pixel of frame 1")
+    seq = []
     prev = None
-    worst_t = worst_inc = worst_self = 0.0
-    horizon = None                                                      # K*: first frame where the reference is unstable under a 1-LSB input change
-    slices_at_horizon = None
+    worst_t = worst_inc = 0.0
     for k in range(nframes):
         d, c = frames26[k]
-        p = mine.process_frame(d, c, k); rt.process(d, c, k)
-        Ra, ta, ga, wa = p.as_tuple(); Rb, tb, gb, wb = rt.pose()
-        if rp is not None:
-            dp = d
-            if k == 1:
-                dp = d.copy(); dp[ROWS // 2, COLS // 2] += 1
-            rp.process(dp, c, k)
-            _, _, gp, wp = rp.pose()
-            self_dev = float(np.abs(gp - gb).max())
-            if horizon is None and (self_dev > 2e-5 or not (wp == wb).all()):
-                horizon = k; slices_at_horizon = n_slices
-                print(f"stable horizon K* = {k}: the reference moved {self_dev:.2e} m under a 1-LSB change of one depth pixel of frame 1")
-            if horizon is None:
-                worst_self = max(worst_self, self_dev)
-        stable = horizon is None
+        pm = mine.process_frame(d, c, k)
+        Ra, ta, ga, wa = pm.as_tuple()
+        gp = G[p + "poses"][k]
+        Rb, tb, gb, wb = gp[:9].reshape(3, 3), gp[9:12], gp[12:15], gp[15:18].astype(np.int32)
+        stable = horizon is None or k < horizon
         # ---- 1. poses ----
         dt = float(np.abs(ta - tb).max())
         if odometry == 0:
@@ -150,63 +173,29 @@ def test_baseline_config_512_live_replay_exact(built, frames26, odometry, nframe
             assert dt <= tol and rot_angle(Ra, Rb) <= tol, (odometry, k, dt, rot_angle(Ra, Rb))
             assert np.abs(ga - gb).max() <= tol
         prev = (ga.copy(), gb.copy())
-        # ---- 2./3. replay this frame with the reference's operators on the product's pose ----
-        dd = torch.from_numpy(d.view(np.int16)).cuda(); cc = torch.from_numpy(c).cuda()
-        ref.bilateral(dd, fb, ROWS, COLS); ref.vmap(fb, vm, ROWS, COLS, intr); ref.nmap(vm, nm, ROWS, COLS)
         # the product's fused front end (kt_frontend.cu) against the reference's operators on this frame: filtered depth, vertex and
         # normal maps of level 0, bit for bit (NaNs in the same places)
         # (values compared as floats: a normal component that is exactly zero may carry either sign -- x - x and 0 * y products, invisible to
         # every consumer)
-        assert np.array_equal(mine.download_map(4, 0), fb.cpu().numpy().view(np.uint16)), (odometry, k, "bilateral")
-        assert np.array_equal(mine.download_map(0, 0), vm.cpu().numpy().reshape(3, ROWS, COLS), equal_nan=True), (odometry, k, "vmap")
-        assert np.array_equal(mine.download_map(1, 0), nm.cpu().numpy().reshape(3, ROWS, COLS), equal_nan=True), (odometry, k, "nmap")
-        for axis in range(3):                                           # x, then y, then z (.cpp:675-831)
-            n = int(wa[axis]) - cur[axis]
-            if n == 0:
-                continue
-            assert abs(n) == cfg.voxel_shift
-            box = shift_box(axis, n, cfg.overlap)
-            cnt = ref.extract(ts, vs, ob, cap, vwrap_nonneg(cur), cs, box, 1, cur)
-            want = canon(ob.cpu().numpy().view(refbind.POINT_DTYPE)[:cnt])
-            pts, dim, cam_t = mine.get_slice(n_slices)
-            got = canon(pts)
-            assert dim == (2 * axis + (0 if n > 0 else 1))
-            assert got.shape == want.shape and (got == want).all(), (odometry, k, axis, got.shape, want.shape)
-            slice_points += len(pts)
-            ref.clear(axis, 1 if n < 0 else 0, ts, cs, cur[axis], cur[axis] + n)
-            cur[axis] += n
-            n_slices += 1
-            shifted_frames.append(k)
+        fe = G["frontend"][k]
+        assert digest(mine.download_map(4, 0).view(np.int16)) == fe[0], (odometry, k, "bilateral")
+        assert digest(mine.download_map(0, 0), "values") == fe[1], (odometry, k, "vmap")
+        assert digest(mine.download_map(1, 0), "values") == fe[2], (odometry, k, "nmap")
         Rinv, tint, wint = mine.last_integrate()
-        assert list(wint) == (vwrap_nonneg(cur) if k > 0 else [0, 0, 0])
-        ref.integrate(dd, ROWS, COLS, intr, vs, Rinv, tint, trunc, ts, cs, wint, cc, nm, 1, ds)
+        seq.append(np.concatenate([wa, Rinv.reshape(-1), tint, wint]).astype(np.float64))
+    seq = np.array(seq)
+    # ---- 2./3. replay the product's own pose sequence: its volume and its slices, exactly ----
+    ts, cs, cur, slabs = _replay(frames26, seq, cfg, trunc)
+    n_slices = len(slabs)
     assert mine.num_slices() == n_slices
-    if odometry == 0:
-        assert horizon is None or horizon >= 40, horizon               # the synthetic scene is well conditioned for at least 40 frames
-        n_cmp = n_slices if horizon is None else slices_at_horizon
-    else:
-        n_cmp = n_slices
-        assert rt.num_slices() == n_slices
-    assert n_slices >= 1, "the run must cross the -t 14 shift threshold"
-    if odometry == 0:
-        assert n_slices >= 4, n_slices
-        assert n_cmp >= 3, n_cmp                                        # three shifts inside the stable horizon
-        # 3b. the leaving slabs of this stream are mostly free space (the camera moves away from what it saw), so a slab that certainly
-        # contains surface is extracted as well: 30 z planes around the room's back wall, on the replayed volume at the final cyclic
-        # offset, product operator against the reference's extractCloudSlice -- the same multiset of points.
-        import kintinuous_b200 as kb2
-        wall = int((5.5 - cur[2] * SIZE / V) / (SIZE / V))
-        box = (0, V, 0, V, max(0, wall - 15), min(V - 1, wall + 15))
-        oa = torch.zeros(cap * 32, dtype=torch.uint8, device="cuda")
-        n_b = ref.extract(ts, vs, ob, cap, vwrap_nonneg(cur), cs, box, 1, cur)
-        n_a = kb2.ops.extract_slice(ts, vs, V, oa, cap, vwrap_nonneg(cur), cs, box, 1, tuple(cur))
-        assert n_a == n_b and n_a > 20000, (n_a, n_b, box)
-        assert (canon(oa.cpu().numpy().view(refbind.POINT_DTYPE)[:n_a]) == canon(ob.cpu().numpy().view(refbind.POINT_DTYPE)[:n_b])).all()
-        print(f"back-wall slab {box}: {n_a} points, multiset identical to the reference's extraction")
-    for i in range(n_cmp):                                              # the reference tracker's own slices: same events, same sizes to 1 %
-        a, dim_a, _ = mine.get_slice(i); b, dim_b, _ = rt.get_slice(i)
-        assert dim_a == dim_b and abs(len(a) - len(b)) <= 0.01 * len(b) + 5, (i, len(a), len(b))
-    torch.cuda.synchronize()
+    slice_points = 0
+    for i, (k, axis, n, want) in enumerate(slabs):
+        pts, dim, cam_t = mine.get_slice(i)
+        got = canon(pts)
+        assert dim == (2 * axis + (0 if n > 0 else 1))
+        assert got.shape == want.shape and (got == want).all(), (odometry, k, axis, got.shape, want.shape)
+        slice_points += len(pts)
+    shifted_frames = [s[0] for s in slabs]
     ta_, ca_ = mine.export_volume()
     tr_ = ts.cpu().numpy().reshape(V, V, V); cr_ = cs.cpu().numpy().reshape(V, V, V, 4)
     touched = int((cr_[..., 3] != 0).sum())
@@ -216,18 +205,55 @@ def test_baseline_config_512_live_replay_exact(built, frames26, odometry, nframe
         idx = np.argwhere((ca_ != cr_).any(-1))
         print("colour mismatches:", bad_c, "first", idx[:8].tolist(), "mine", ca_[tuple(idx[:8].T)].tolist(), "replay", cr_[tuple(idx[:8].T)].tolist(),
               "z range", idx[:, 0].min(), idx[:, 0].max(), "y range", idx[:, 1].min(), idx[:, 1].max(), "x range", idx[:, 2].min(), idx[:, 2].max())
-    assert bad_t == 0 and bad_c == 0, (odometry, "voxels differing from the replay with the reference's operators", bad_t, bad_c, touched)
-    # the reference tracker's own volume, for the record: differences come only from its 1e-6 different poses
-    tb_, cb_ = rt.export_volume()
-    dlsb = np.abs(ta_.astype(np.int32) - tb_.astype(np.int32))[cb_[..., 3] != 0]
+    assert bad_t == 0 and bad_c == 0, (odometry, "voxels differing from the replay", bad_t, bad_c, touched)
+    del ta_, ca_, tr_, cr_
+    # ---- the replay's operators are the reference's: replaying the recorded pose sequence gives the reference replay's results ----
+    rec = G[p + "replay_seq"]
+    if not np.array_equal(seq, rec):
+        del ts, cs
+        torch.cuda.empty_cache()
+        ts, cs, cur, slabs = _replay(frames26, rec, cfg, trunc)
+    shifts = G[p + "shifts"]
+    assert len(slabs) == len(shifts)
+    for i, (k, axis, n, pts) in enumerate(slabs):
+        assert [k, axis, n, len(pts)] == shifts[i].tolist() and digest(pts) == G[p + f"shift{i}"][0], (odometry, i)
+    assert [digest(ts), digest(cs)] == G[p + "replay_volume"].tolist(), (odometry, "replay volume differs from the reference's")
+    if odometry == 0:
+        n_cmp = n_slices if horizon is None else sum(1 for k in shifted_frames if k < horizon)
+    else:
+        n_cmp = n_slices
+        assert len(G[p + "slices"]) == n_slices
+    assert n_slices >= 1, "the run must cross the -t 14 shift threshold"
+    if odometry == 0:
+        assert horizon is None or horizon >= 40, horizon               # the synthetic scene is well conditioned for at least 40 frames
+        assert n_slices >= 4, n_slices
+        assert n_cmp >= 3, n_cmp                                        # three shifts inside the stable horizon
+        # 3b. the leaving slabs of this stream are mostly free space (the camera moves away from what it saw), so a slab that certainly
+        # contains surface is extracted as well: 30 z planes around the room's back wall, on the replayed volume at the final cyclic
+        # offset, product operator against the reference's extractCloudSlice -- the same multiset of points.
+        wall = int((5.5 - cur[2] * SIZE / V) / (SIZE / V))
+        box = (0, V, 0, V, max(0, wall - 15), min(V - 1, wall + 15))
+        assert list(box) == G[p + "backwall"][:6].tolist()
+        cap = 3 * ROWS * COLS
+        oa = torch.zeros(cap * 32, dtype=torch.uint8, device="cuda")
+        n_a = kb.ops.extract_slice(ts, [SIZE] * 3, V, oa, cap, vwrap_nonneg(cur), cs, box, 1, tuple(cur))
+        n_b = int(G[p + "backwall"][6])
+        assert n_a == n_b and n_a > 20000, (n_a, n_b, box)
+        assert digest(canon_points(oa[:n_a * 32])) == G[p + "backwall_digest"][0]
+        print(f"back-wall slab {box}: {n_a} points, multiset identical to the reference's extraction")
+    for i in range(n_cmp):                                              # the reference tracker's own slices: same events, same sizes to 1 %
+        a, dim_a, _ = mine.get_slice(i); dim_b, n_b = G[p + "slices"][i]
+        assert dim_a == dim_b and abs(len(a) - n_b) <= 0.01 * n_b + 5, (i, len(a), n_b)
+    # the reference tracker's own volume, for the record (a seeded sample of its touched voxels): differences come only from its 1e-6
+    # different poses
+    ta_, _ = mine.export_volume(color=False)
+    dlsb = np.abs(ta_.reshape(-1)[G[p + "ref_vol_idx"]].astype(np.int32) - G[p + "ref_vol_tsdf"].astype(np.int32))
     frac = float((dlsb <= 1).mean())
-    print(f"cfg odometry={odometry}: stable horizon {horizon}, worst |dt| {worst_t:.3e} m (reference vs its 1-LSB-perturbed self: {worst_self:.3e} m), worst per-frame increment difference {worst_inc:.3e} m; {nframes} frames, shifts at {shifted_frames} ({slice_points} slice points), touched {touched}, replay mismatches 0/0, "
-          f"vs reference tracker: {frac:.6f} of touched voxels within 1 LSB, worst {int(dlsb.max())} LSB")
+    print(f"cfg odometry={odometry}: stable horizon {horizon}, worst |dt| {worst_t:.3e} m (reference vs its 1-LSB-perturbed self: {float(G[p + 'worst_self']):.3e} m), worst per-frame increment difference {worst_inc:.3e} m; {nframes} frames, shifts at {shifted_frames} ({slice_points} slice points), touched {touched}, replay mismatches 0/0, "
+          f"vs reference tracker: {frac:.6f} of sampled touched voxels within 1 LSB, worst {int(dlsb.max())} LSB")
     if odometry == 0 and horizon is None:
         assert frac >= 0.999
-    mine.close(); rt.close()
-    if rp is not None:
-        rp.close()
+    mine.close()
 
 
 _PI_SCRIPT = r"""
@@ -318,56 +344,50 @@ def test_wrap_beyond_one_volume_length(built):
     """voxelWrap grows without bound while the volume travels in +x/+y/+z (vWrapCopy only folds negative values,
     KintinuousTracker.cpp:1075-1085); the reference kernels reduce it with % VOLUME per access.  Offsets > V, a multiple of V, and
     negative ones must address the same storage as their residue: integrate, raycast, extract and clear against the reference's
-    kernels on identical buffers, bit-exact."""
+    kernels on identical buffers, bit-exact (by digest: tests/golden/ref_ops_live.npz)."""
     import torch
     import kintinuous_b200 as kb
     from kintinuous_b200 import synth
-    from oracle import refbind
+    from oracle.golden import digest, canon_points
+    live = np.load(os.path.join(GOLDEN, "ref_ops_live.npz"))
     Vs = 256
-    if not refbind.RefCuda.available(Vs):
-        pytest.skip("oracle/_ref not present")
-    ref = refbind.RefCuda(Vs)
     ops = kb.ops
     rows, cols = 120, 160
     intr = np.array(synth.intrinsics(cols, rows), np.float32)
     d, c = synth.render(0, cols, rows)
     dd = torch.from_numpy(d.view(np.int16)).cuda(); cc = torch.from_numpy(c).cuda()
-    fb = torch.zeros((rows, cols), dtype=torch.int16, device="cuda"); ref.bilateral(dd, fb, rows, cols)
+    fb = torch.zeros((rows, cols), dtype=torch.int16, device="cuda"); ops.bilateral(dd, fb, rows, cols)
     vm = torch.zeros((3 * rows, cols), dtype=torch.float32, device="cuda"); nm = torch.zeros_like(vm)
-    ref.vmap(fb, vm, rows, cols, intr); ref.nmap(vm, nm, rows, cols)
+    ops.create_vmap(intr, fb, vm, rows, cols); ops.create_nmap(vm, nm, rows, cols)
+    assert [digest(fb), digest(vm, "map"), digest(nm, "map")] == live["wrap_inputs"].tolist()      # the reference's input maps
     vs = [SIZE] * 3; trunc = 0.06
     ang = 0.05
     R = np.array([[np.cos(ang), 0, np.sin(ang)], [0, 1, 0], [-np.sin(ang), 0, np.cos(ang)]], np.float32)
     Rinv = np.linalg.inv(R.astype(np.float64)).astype(np.float32)
     t = np.array([3.02, 2.99, 3.01], np.float32)
-    for wrap in ((Vs + 88, 2 * Vs + 3, 3 * Vs - 1), (Vs, 2 * Vs, 0), (5 * Vs + 17, 31, Vs + 200)):
+    for i, wrap in enumerate(((Vs + 88, 2 * Vs + 3, 3 * Vs - 1), (Vs, 2 * Vs, 0), (5 * Vs + 17, 31, Vs + 200))):
+        want = live["wrap_steps"][i]
         ta = torch.zeros(Vs ** 3, dtype=torch.int16, device="cuda"); ca = torch.zeros(Vs ** 3 * 4, dtype=torch.uint8, device="cuda")
-        tb = torch.zeros_like(ta); cb = torch.zeros_like(ca)
         ds = torch.zeros((rows, cols), dtype=torch.float32, device="cuda")
         ops.integrate(dd, rows, cols, intr, vs, Rinv, t, trunc, ta, ca, Vs, wrap, cc, nm, 1, ds)
-        ref.integrate(dd, rows, cols, intr, vs, Rinv, t, trunc, tb, cb, wrap, cc, nm, 1, ds)
         torch.cuda.synchronize()
-        assert int((cb.view(-1, 4)[:, 3] != 0).sum()) > 10000
-        assert bool((ta == tb).all()) and bool((ca == cb).all()), wrap
+        assert int((ca.view(-1, 4)[:, 3] != 0).sum()) > 10000
+        assert digest(ta) == want[0] and digest(ca) == want[1], wrap
         va = torch.zeros_like(vm); na = torch.zeros_like(vm); xa = torch.zeros((rows, cols, 4), dtype=torch.uint8, device="cuda")
-        vb = torch.zeros_like(vm); nb = torch.zeros_like(vm); xb = torch.zeros_like(xa)
         ops.raycast(intr, R, t, trunc, vs, ta, Vs, va, na, rows, cols, wrap, xa, ca)
-        ref.raycast(intr, R, t, trunc, vs, tb, vb, nb, rows, cols, wrap, xb, cb)
         torch.cuda.synchronize()
-        assert torch.equal(va.view(torch.int32), vb.view(torch.int32)) and torch.equal(na.view(torch.int32), nb.view(torch.int32)) and torch.equal(xa, xb), wrap
+        assert digest(va) == want[2] and digest(na) == want[3] and digest(xa) == want[4], wrap
         cap = 400000
-        oa = torch.zeros(cap * 32, dtype=torch.uint8, device="cuda"); ob = torch.zeros_like(oa)
+        oa = torch.zeros(cap * 32, dtype=torch.uint8, device="cuda")
         box = (0, Vs, 0, Vs, 225, 242)                             # the back wall of the room (z = 5.5 m -> voxel 234)
         real = tuple(int(w) for w in wrap)
         n_a = ops.extract_slice(ta, vs, Vs, oa, cap, wrap, ca, box, 1, real)
-        n_b = ref.extract(tb, vs, ob, cap, wrap, cb, box, 1, real)
-        assert n_a == n_b and n_a > 100
-        assert (canon(oa.cpu().numpy().view(refbind.POINT_DTYPE)[:n_a]) == canon(ob.cpu().numpy().view(refbind.POINT_DTYPE)[:n_b])).all()
+        assert n_a == int(live["wrap_counts"][i][0]) and n_a > 100
+        assert digest(canon_points(oa[:n_a * 32])) == want[5], wrap
         for axis in range(3):
             ops.clear_volume(axis, 0, ta, ca, Vs, wrap[axis], wrap[axis] + 14)
-            ref.clear(axis, 0, tb, cb, wrap[axis], wrap[axis] + 14)
         torch.cuda.synchronize()
-        assert bool((ta == tb).all()) and bool((ca == cb).all()), ("clear", wrap)
+        assert digest(ta) == want[6] and digest(ca) == want[7], ("clear", wrap)
 
 
 def test_tracker_tracks_ground_truth_across_repeated_shifts(built):

@@ -75,7 +75,8 @@ def main():
     g["vol_idx"] = nz.astype(np.int32); g["vol_tsdf"] = tsdf.reshape(-1)[nz]; g["vol_color"] = col.reshape(-1, 4)[nz]
     va = torch.zeros_like(vm); na = torch.zeros_like(vm); cc = torch.zeros((rows, cols, 4), dtype=torch.uint8, device="cuda")
     ref.raycast(intr, R1, t1, trunc, vs, ts, va, na, rows, cols, wrap, cc, cs)
-    g["raycast_v"] = va.cpu().numpy(); g["raycast_n"] = na.cpu().numpy(); g["raycast_c"] = cc.cpu().numpy()
+    # kept in a file of their own: every golden file stays under 1 MB
+    np.savez_compressed(os.path.join(OUT, "ops_160x120_raycast.npz"), raycast_v=va.cpu().numpy(), raycast_n=na.cpu().numpy(), raycast_c=cc.cpu().numpy())
     cap = 400000
     ob = torch.zeros(cap * 32, dtype=torch.uint8, device="cuda")
     real = (14, 3, 250 - V)
